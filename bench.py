@@ -5,10 +5,13 @@ A "step" = one pass of the hot path over one batch of synthetic problems: DualMu
 interior-point solve (rounds of k_pk_eval [K1] / k_pk_sweep [K3] / k_pk_step [K4], then the persistent tail kernel) of
 ParkingSignedDist for B randomised start poses.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU, NCCL); the batch is sharded by rank (weak scaling: B per GPU),
 nothing is exchanged on the solve path, one all-reduce carries the counters.  Rank 0 prints ONE JSON line.
+
+--dump-outputs DIR: rank 0 writes what the solver returned in the last timed step as DIR/<name>.npy (float64; see dump_outputs).
+The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
   value      converged trajectories / s, inputs resident in HBM, device time from CUDA events on the library's
              stream (max over ranks)
@@ -273,6 +276,9 @@ def gpu_arm(args):
         dev_s += step_dev()
     barrier()
     wall_s = time.perf_counter() - t_wall0
+    if args.dump_outputs and rank == 0:      # before the e2e and profiling solves below reuse the device buffers
+        dump_outputs(args.dump_outputs, dict(xp=dout["xp"], up=dout["up"], ts=dout["ts"], lp=dout["lp"], np=dout["np"], sl=dout["sl"],
+                                             exitflag=dflag, iters=dit, kkt_err=dout["err"]))
     conv = int(dflag.sum().item()); it_sum = int(dit.sum().item()); it_max = int(dit.max().item())
     evals = it_sum + B
     # ---- end-to-end through the host-pointer C-ABI ----
@@ -472,6 +478,8 @@ def gpu_arm_other(args):
         e2e_s += time.perf_counter() - t0
         dev_s += r["time"]; conv += ok(r); its += int(r["iters"].sum())
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {k: v for k, v in r.items() if k != "time"})
     sampler.stop = True; sampler.join()
     stats = torch.tensor([dev_s, e2e_s], dtype=torch.float64, device="cuda")
     cnt = torch.tensor([conv, its], dtype=torch.float64, device="cuda")
@@ -491,6 +499,24 @@ def gpu_arm_other(args):
         emit(line)
     if dist is not None:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes one step's outputs (arrays or tensors with the problem index on axis 0) as out_dir/<name>.npy in float64.  When all
+    of them would exceed DUMP_BYTES, a sample of the problems drawn with a fixed seed is written instead, the same for every run
+    with the same batch; problem.npy holds the batch indices of the rows written (all of them when nothing was dropped)."""
+    arrays = {k: np.asarray(v.cpu() if hasattr(v, "cpu") else v, dtype=np.float64) for k, v in arrays.items()}
+    B = len(next(iter(arrays.values())))
+    per_problem = 8 * (1 + sum(a[0].size for a in arrays.values()))
+    n = min(B, (DUMP_BYTES - 1024 * (len(arrays) + 1)) // per_problem)          # 1 KB per file for the .npy header
+    idx = np.arange(B) if n == B else np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "problem.npy"), idx.astype(np.float64))
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a[idx])
 
 
 _OUT_FD = None
@@ -524,7 +550,13 @@ def main():
                     help="weak (default, the headline): --batch problems PER GPU; strong: --batch problems in total, sharded over the GPUs")
     ap.add_argument("--workload", default="reverse", choices=["reverse", "parallel", "parallel4", "quadcopter", "dist", "fixed"],
                     help="reverse = BASELINE config 2 (the headline line, default); the others print a secondary line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the solver outputs of the last timed step to DIR/<name>.npy (GPU arms; at most 64 MB, sampled by problem above that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arms; the reference arm returns none")
     if args.impl == "reference":
         reference_arm(args)
     elif args.workload != "reverse":
